@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the registrators/ hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One *alignment* is BASELINE.json configs[1]: a synthetic 64-beam 120 000-point scan against a
 500 000-point submap (106 784 target points with normals after the caller-side CalculateNormals),
@@ -11,10 +11,14 @@ rebuild.  One *step* is a BATCH of --batch (64) such alignments per GPU — BASE
 configs[3]'s per-GPU share (512 pairs on 8 GPUs) — pushed through the batched entry point
 sm_align_pairs by --host-threads (2) host threads over --pipelines (16) matcher instances.
 
-* `value`  : alignments/s, clouds already resident in HBM (device pointers), median of 3 windows
-             of K steps, device time (CUDA events), max over ranks, pose all-gather included.
+* `value`  : alignments/s, clouds already resident in HBM (device pointers), K timed steps (one window
+             unless --windows splits them; then the median per-step time), device time (CUDA events), max
+             over ranks, pose all-gather included.
 * `e2e`    : the same through host buffers (pinned host memory -> H2D inside the timed region,
-             result records read back, all-gather included).
+             result records read back, all-gather included), another K timed steps.
+* --dump-outputs DIR : the rcs, poses and scores that the last timed step of each path returned
+             (`icp_*`, `icp_e2e_*`, `ndt_*`, `ndt_gicp_*`) as float64 .npy files; the inputs are seeded, so
+             they are the same from run to run.
 * roofline : dominant kernel (transform + k-NN), algorithmic bytes of SURVEY.md section 8d over the
              CUDA-event time of its launches, measured here with one alignment in flight; the
              16-in-flight regime of `value` is reported beside it (kernels of different alignments
@@ -158,14 +162,27 @@ def oracle_module(threads):
 
 def cpu_time_alignments(O, src, tp, tn, min_reps, max_seconds):
     """Full oracle alignments (fixed 30 iterations) until `min_reps` are done and, beyond that,
-    while less than `max_seconds` have been spent."""
+    while less than `max_seconds` have been spent.  Returns (seconds per alignment, the last alignment's result)."""
     ts = []
     while len(ts) < min_reps or (sum(ts) < max_seconds and len(ts) < 4 * min_reps):
         t0 = time.perf_counter()
         r = O.icp_fast_align(src, tp, tn, max_iteration=ITERATIONS, disable_convergence_check=True)
         ts.append(time.perf_counter() - t0)
         assert r["rc"] == 1 and r["iterations"] == ITERATIONS
-    return ts
+    return ts, r
+
+
+def window_steps(steps, windows):
+    """The `steps` timed steps split into at most `windows` windows whose sizes differ by at most one."""
+    w = min(windows, steps)
+    return [steps // w + (k < steps % w) for k in range(w)]
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: one float64 .npy per returned array."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 def workload_config(n_target, batch):
@@ -187,7 +204,9 @@ def run_reference(args, rank, world):
     src, sub, _ = make_workload(0)
     tp, tn = O.calculate_normals(sub)
     cpu_time_alignments(O, src, tp, tn, max(1, min(args.warmup, 2)), 0.0)
-    ts = cpu_time_alignments(O, src, tp, tn, args.steps, 0.0)[:args.steps]
+    ts, r = cpu_time_alignments(O, src, tp, tn, args.steps, 0.0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"icp_ok": [r["rc"]], "icp_poses": r["result"][None], "icp_scores": [r["score"]]})
     total = float(np.sum(ts))
     value = len(ts) / total
     cores = O.num_threads()
@@ -294,10 +313,18 @@ def main():
     ap.add_argument("--pipelines", "--inflight", type=int, default=16, dest="pipelines",
                     help="matcher instances (= alignments in flight) per GPU")
     ap.add_argument("--host-threads", type=int, default=2, help="host threads that drive the pipelines")
-    ap.add_argument("--windows", type=int, default=3, help="timed windows of --steps steps; the median is reported")
+    ap.add_argument("--windows", type=int, default=1,
+                    help="timed windows the --steps steps are split into; the median per-step time is reported "
+                         "(each window adds ~2 ms of ramp-up and drain on a B200 at 1000 W, so shorter windows "
+                         "lower the figure)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the Ndt / NdtWithGicp records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each timed path returned as DIR/<name>.npy (float64; "
+                         "rank 0's pairs), so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.windows < 1:
+        ap.error("--steps and --windows must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -371,7 +398,8 @@ def main():
         """`steps` batches of B alignments through sm_align_pairs: host thread j drives the pipelines
         j, j+T, ... with the pairs j, j+T, ... of the batch.  Device time of the whole region: an
         event before (every pipeline stream waits on it) and one after (it waits on every pipeline),
-        plus the all-gather of the last batch's poses."""
+        plus the all-gather of the last batch's poses.  Returns (ms, what the last step returned for the
+        batch: rcs, poses, scores in batch order)."""
         e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
         errors, last = [], [None] * T
         gate = threading.Barrier(T + 1)
@@ -383,8 +411,7 @@ def main():
             try:
                 gate.wait()
                 for _ in range(steps):
-                    rcs, res, sc = smb.AlignPairs(ms, mine)
-                    last[j] = (res, sc)
+                    last[j] = smb.AlignPairs(ms, mine)
             except Exception as e:  # noqa: BLE001
                 errors.append(e)
 
@@ -404,10 +431,11 @@ def main():
             ev = torch.cuda.Event(); ev.record(s); tstream.wait_event(ev)
         e1.record(tstream)
         e1.synchronize()
-        res = np.concatenate([x[0] for x in last if x is not None])
-        sc = np.concatenate([x[1] for x in last if x is not None])
+        rcs, res, sc = np.empty(B), np.empty((B, 4, 4)), np.empty(B)
+        for j, (rcs_j, res_j, sc_j) in enumerate(last):
+            rcs[j::T], res[j::T], sc[j::T] = rcs_j, res_j, sc_j
         gather_poses(res, sc)                 # once per window, inside the reported time
-        return e0.elapsed_time(e1) + (gather_ms[-1] if world > 1 else 0.0), res
+        return e0.elapsed_time(e1) + (gather_ms[-1] if world > 1 else 0.0), (rcs, res, sc)
 
     # ---- warm-up (graphs captured, allocations done, all-gather warmed) -------------------------
     run_steps(args.warmup, False)
@@ -420,23 +448,27 @@ def main():
     barrier()
     gather_ms.clear()
     t_mark0 = sampler.mark() if sampler else None
+    windows = window_steps(args.steps, args.windows)
     # ---- timed: device-resident inputs -------------------------------------------------------
     win_dev = []
-    for _ in range(args.windows):
+    for n in windows:
         barrier()
-        ms, _ = run_steps(args.steps, False)
+        ms, dev_out = run_steps(n, False)
         barrier()
         win_dev.append(max_over_ranks(ms))
     # ---- timed: host buffers through the public API (H2D inside) ---------------------------
     win_e2e = []
-    for _ in range(args.windows):
+    for n in windows:
         barrier()
-        ms, _ = run_steps(args.steps, True)
+        ms, e2e_out = run_steps(n, True)
         barrier()
         win_e2e.append(max_over_ranks(ms))
     t_mark1 = sampler.mark() if sampler else None
-    ms_dev_total = float(np.median(win_dev))
-    ms_e2e_total = float(np.median(win_e2e))
+    outputs = {}
+    for prefix, (rcs, res, sc) in (("icp", dev_out), ("icp_e2e", e2e_out)):
+        outputs.update({f"{prefix}_ok": rcs, f"{prefix}_poses": res, f"{prefix}_scores": sc})
+    ms_dev_step = float(np.median([ms / n for ms, n in zip(win_dev, windows)]))
+    ms_e2e_step = float(np.median([ms / n for ms, n in zip(win_e2e, windows)]))
     gpu_launches = per_align_launches * B * args.steps
     allgather_incl_wait_ms = float(np.median(gather_ms)) if gather_ms else 0.0
     allgather_ms = 0.0
@@ -494,9 +526,8 @@ def main():
     w0.InitWithXml({"profile_kernels": 0})
     clocks = sampler.stop(t_mark0, t_mark1) if sampler else None
 
-    n_align = args.steps * B
-    value = n_align * world / (ms_dev_total * 1e-3)
-    e2e_value = n_align * world / (ms_e2e_total * 1e-3)
+    value = B * world / (ms_dev_step * 1e-3)
+    e2e_value = B * world / (ms_e2e_step * 1e-3)
     knn_ms = prof["knn"] / prof["n"] / ITERATIONS          # average launch duration
     peaks = {}
     try:
@@ -527,7 +558,7 @@ def main():
                 "traversal_inclusive_frac": (382 * N_SOURCE / (knn_ms * 1e-3) / 1e9) / peak}
 
     cfg = workload_config(d0.nt, B)
-    cfg.update({"pipelines_per_gpu": P, "host_threads": T, "windows": args.windows,
+    cfg.update({"pipelines_per_gpu": P, "host_threads": T, "windows": len(windows), "steps_per_window": windows,
                 "entry_point": "sm_align_pairs (one call per host thread and step)",
                 "l2": f"{P} distinct pairs in flight per GPU (combined working set ~{25 * P} MB vs 126 MB L2), every "
                       "alignment re-uploads / re-reads its clouds and rebuilds its tree; the latency figures flush "
@@ -535,11 +566,11 @@ def main():
                 "timed_window_ms": {"device_resident": win_dev, "host_buffers": win_e2e}})
     out = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
-        "warmup": args.warmup, "ms_per_step": ms_dev_total / args.steps,
+        "warmup": args.warmup, "ms_per_step": ms_dev_step,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
         "data": "synthetic", "config": cfg,
         "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": d0.h2d_bytes * B,
-                "d2h_bytes_per_step": (128 + 400) * B, "ms_per_step": ms_e2e_total / args.steps},
+                "d2h_bytes_per_step": (128 + 400) * B, "ms_per_step": ms_e2e_step},
         "latency": {"ms_per_alignment_device": ms_lat_dev, "ms_per_alignment_host_buffers": ms_lat_host,
                     "in_flight": 1, "icp_iterations_per_s": ITERATIONS / (iter_ms * 1e-3)},
         "gpu_launches": gpu_launches, "clocks": clocks, "roofline": roofline,
@@ -553,7 +584,7 @@ def main():
     # ---- extra: configs[2] (Ndt) and configs[4] (NdtWithGicp, sharded, pose all-gather) ----------
     if not args.no_extra:
         try:
-            out["extra"] = run_extra(args, smb, torch, dist, parallel, dev, rank, local_rank, world, P)
+            out["extra"] = run_extra(args, smb, torch, dist, parallel, dev, rank, local_rank, world, P, outputs)
         except Exception as e:  # noqa: BLE001
             # the headline measurement above is complete: with one rank a failure of the side records must not
             # lose it (with several ranks the others are inside collectives, so the error has to propagate)
@@ -571,6 +602,8 @@ def main():
             if isinstance(rec, dict):
                 rec.pop("result_check", None)
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(out), flush=True)
     # orderly teardown: drain the GPU and destroy the engine handles before the interpreter
     # (and torch's CUDA context) goes away
@@ -589,7 +622,7 @@ def cpu_legs(out, d0, res_check):
     benchmarked configuration and the oracle beside the extra records: rank 0 at N = 1 only."""
     threads, res = cpu_threads()
     O = oracle_module(threads)
-    ts = cpu_time_alignments(O, d0.src, d0.tp, d0.tn, 3, 10.0)
+    ts, _ = cpu_time_alignments(O, d0.src, d0.tp, d0.tn, 3, 10.0)
     # parity spot check of the benchmarked configuration against the oracle
     o = O.icp_fast_align(d0.src, d0.tp, d0.tn, max_iteration=ITERATIONS, disable_convergence_check=True)
     E = np.linalg.inv(o["result"]) @ res_check
@@ -602,7 +635,7 @@ def cpu_legs(out, d0, res_check):
         "sample": f"{len(ts)} full alignments of the same workload (30 fixed iterations, tree rebuilt each "
                   f"time), one at a time, OpenMP over queries with {cores} threads (one per usable physical core)"}
     O.set_num_threads(6)                  # the reference's own hard-coded thread count (ndt.cc:32)
-    ts6 = cpu_time_alignments(O, d0.src, d0.tp, d0.tn, 2, 6.0)
+    ts6, _ = cpu_time_alignments(O, d0.src, d0.tp, d0.tn, 2, 6.0)
     out["cpu_baseline"]["six_threads"] = {"value": len(ts6) / float(np.sum(ts6)), "unit": UNIT, "cores": 6,
                                           "sample": f"{len(ts6)} alignments"}
     O.set_num_threads(threads)
@@ -610,9 +643,10 @@ def cpu_legs(out, d0, res_check):
         cpu_extra(O, out["extra"])
 
 
-def run_extra(args, smb, torch, dist, parallel, dev, rank, local_rank, world, pairs_per_rank):
+def run_extra(args, smb, torch, dist, parallel, dev, rank, local_rank, world, pairs_per_rank, outputs):
     """Ndt (configs[2]) and NdtWithGicp (configs[4]: 2048 loop-closure candidate pairs sharded over the
-    ranks, poses all-gathered) on the same clouds: float scan + raw 500k submap."""
+    ranks, poses all-gathered) on the same clouds: float scan + raw 500k submap.  What the last timed batch
+    of each returned goes into `outputs`."""
     from staticmapping_b200 import InnerCloud
     npairs = 4
     clouds = []
@@ -646,6 +680,7 @@ def run_extra(args, smb, torch, dist, parallel, dev, rank, local_rank, world, pa
             oks, res = smb.AlignBatch(ms_, guesses)
             all_res.extend(res); all_sc.extend(m.GetFitnessScore() for m in ms_)
             done += npairs
+        outputs.update({f"{name}_ok": oks, f"{name}_poses": res, f"{name}_scores": all_sc[-npairs:]})
         ag_ms = 0.0
         if world > 1:
             rec = parallel.pack_poses(all_res, all_sc)                 # every pose of the shard: 136 B per pair

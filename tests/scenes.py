@@ -9,10 +9,14 @@ from staticmapping_b200 import synth
 
 
 def se3_error(A, B):
-    """(translation error [m], rotation angle [rad]) between two 4x4 transforms."""
+    """(translation error [m], rotation angle [rad]) between two 4x4 transforms.  The angle is
+    atan2(sin, cos) of the relative rotation: arccos of the trace alone cannot resolve angles below
+    2.1e-8 rad, the angle it returns when the trace is one rounding step below 3."""
     E = np.linalg.inv(A) @ B
-    c = np.clip((np.trace(E[:3, :3]) - 1.0) / 2.0, -1.0, 1.0)
-    return float(np.linalg.norm(E[:3, 3])), float(np.arccos(c))
+    R = E[:3, :3]
+    s = 0.5 * np.linalg.norm([R[2, 1] - R[1, 2], R[0, 2] - R[2, 0], R[1, 0] - R[0, 1]])
+    c = 0.5 * (np.trace(R) - 1.0)
+    return float(np.linalg.norm(E[:3, 3])), float(np.arctan2(s, c))
 
 
 @functools.lru_cache(maxsize=None)
