@@ -274,6 +274,65 @@ inline void CalculateNormalsB200(data::EigenPointCloud* cloud, int device = 0) {
   cloud->normals = nrm.leftCols(m);
 }
 
+// builder::MultiResolutionVoxelMap (builder/multi_resolution_voxel_map.{h,cc}) on the GPU: the map stays on the
+// device across inserts.  Semantics are the reference's run by one thread; output comes in ascending voxel order
+// (include/sm_b200.h lists the deviations).  INTEGRATION.md shows the members of the reference class forwarding here.
+class MultiResolutionVoxelMapB200 {
+ public:
+  explicit MultiResolutionVoxelMapB200(int device = 0, int64_t expected_voxels = 1 << 22)
+      : device_(device), expected_voxels_(expected_voxels) {}
+  ~MultiResolutionVoxelMapB200() { if (handle_) sm_mrvm_destroy(handle_); }
+  MultiResolutionVoxelMapB200(const MultiResolutionVoxelMapB200&) = delete;
+  MultiResolutionVoxelMapB200& operator=(const MultiResolutionVoxelMapB200&) = delete;
+
+  // Initialise (:42-48), from the reference's MrvmSettings (or anything with its field names)
+  template <typename Settings>
+  void Initialise(const Settings& s) {
+    sm_mrvm_settings st;
+    st.output_average = s.output_average; st.output_rgb = s.output_rgb; st.use_max_intensity = s.use_max_intensity;
+    st.prob_threshold = s.prob_threshold; st.low_resolution = s.low_resolution; st.high_resolution = s.high_resolution;
+    st.hit_prob = s.hit_prob; st.miss_prob = s.miss_prob; st.z_offset = s.z_offset;
+    st.max_point_num_in_cell = s.max_point_num_in_cell;
+    if (handle_) sm_mrvm_destroy(handle_);
+    handle_ = nullptr;
+    const int rc = sm_mrvm_create(device_, &st, expected_voxels_, &handle_);
+    CHECK_EQ(rc, 0) << "sm_mrvm_create failed (" << rc << "): invalid MrvmSettings or no CUDA device";
+  }
+
+  void SetOffsetZ(const float& offset) { CHECK_EQ(sm_mrvm_set_offset_z(handle_, offset), 0); }
+
+  // InsertPointCloud (:54-123); origin = the sensor position (x, y, z)
+  void InsertPointCloud(const data::InnerCloudType& cloud, const float* origin) {
+    CHECK(handle_);
+    if (cloud.points.empty()) {                               // "cloud is empty." (:56-59)
+      LOG(ERROR) << "cloud is empty.";
+      return;
+    }
+    const int rc = sm_mrvm_insert(handle_, &cloud.points[0].x, static_cast<int64_t>(cloud.points.size()),
+                                  sizeof(data::InnerPointType), origin);
+    CHECK_GE(rc, 0) << "sm_mrvm_insert failed (" << rc << "): voxel index outside +-2^20 or CUDA failure";
+    if (rc > 0) LOG(ERROR) << rc << " points with a non-finite coordinate dropped";
+  }
+
+  size_t size() const { return handle_ ? static_cast<size_t>(sm_mrvm_size(handle_)) : 0; }
+
+  // OutputToPointCloud (:125-215): {x, y, z, intensity} records (rgb = false, the PointXYZI overload) or
+  // {x, y, z, grey level} (rgb = true, PointXYZRGB with r = g = b = grey)
+  void OutputToPointCloud(float threshold, bool rgb, std::vector<float>* xyzv) const {
+    CHECK(handle_ && xyzv);
+    int64_t m = 0;
+    int rc = sm_mrvm_output(handle_, threshold, rgb ? 1 : 0, nullptr, 0, &m);
+    xyzv->assign(static_cast<size_t>(4 * m), 0.f);
+    if (m > 0) rc = sm_mrvm_output(handle_, threshold, rgb ? 1 : 0, xyzv->data(), m, &m);
+    CHECK_EQ(rc, 0) << "sm_mrvm_output failed (" << rc << ")";
+  }
+
+ private:
+  int device_;
+  int64_t expected_voxels_;
+  sm_mrvm* handle_ = nullptr;
+};
+
 }  // namespace registrator
 }  // namespace static_map
 

@@ -260,6 +260,67 @@ int sm_m2dp(int device, const float* points, int64_t n, int64_t stride_bytes, do
             int32_t t, int32_t p, int32_t q, float* descriptor, int64_t capacity, int32_t* A_out);
 double sm_m2dp_match(const float* P, const float* Q, int64_t n);
 
+/* MultiResolutionVoxelMap (builder/multi_resolution_voxel_map.{h,cc}), the ray-casting occupancy map that
+ * MapBuilder::SaveMaps fills with every frame to write static_map.pcd.  The map lives on the device across inserts.
+ * Points are data::InnerPointType records (x, y, z, intensity, ...) `stride_bytes` (>= 16) apart.
+ * Semantics: those of the reference run by ONE thread.  Per insert, each point casts a Bresenham ray
+ * (common::VoxelCastingBresenham, math.cc:35-95) from origin + (0, 0, z_offset) to its voxel
+ * lround(floor(v / high_resolution)) (float); its end voxel is created if absent and gets one hit (probability,
+ * max_intensity = max(., int(intensity)), the point appended while fewer than max_point_num_in_cell are stored);
+ * every other voxel of the ray gets one miss if it existed before this insert and no earlier point of this insert
+ * ended in it.  Updates are the reference's uint8 -> uint8 maps (float / double expressions of .h:134-140,
+ * .cc:36-40, :63-69).  Deviations from the reference:
+ *   1. InsertPointCloud runs its loop on 10 OpenMP threads (:75-77) with a non-atomic read-modify-write of each
+ *      voxel's probability and unordered point appends (:93-114): its result is not reproducible.  This map
+ *      computes the one-thread result, exactly, whatever the scheduling.
+ *   2. Output is in ascending voxel order (ix, iy, iz), not tbb::concurrent_unordered_map order.
+ *   3. Points with a NaN / inf coordinate are dropped and counted (the reference reaches lround(NaN) and then
+ *      FATAL_CHECK_POINT).
+ *   4. Voxel indices must lie in [-2^20, 2^20) per axis (+-104 km at 0.1 m): an insert with a point or an origin
+ *      outside returns SM_ERR_BAD_ARGUMENT and leaves the map unchanged.
+ * Intensities must be within the int range (the reference converts them with static_cast<int>).
+ * One handle is used by one thread at a time; it owns its CUDA stream.  Every call returns after its device work
+ * has finished. */
+typedef struct sm_mrvm sm_mrvm;
+typedef struct sm_mrvm_settings {   /* MrvmSettings, multi_resolution_voxel_map.h:55-66 (defaults in brackets) */
+  int32_t output_average;           /* [0] one mean point per voxel instead of every stored point */
+  int32_t output_rgb;               /* [0] not read by this API: the caller picks the record type in sm_mrvm_output */
+  int32_t use_max_intensity;        /* [1] */
+  float prob_threshold;             /* [0.6] not read by this API: sm_mrvm_output takes the threshold */
+  float low_resolution;             /* [1.0] unused, like in the reference */
+  float high_resolution;            /* [0.1] voxel size, > 0 */
+  float hit_prob;                   /* [0.55] > 0.5, clamped to [0.501, 0.9] */
+  float miss_prob;                  /* [0.48] < 0.5, clamped to [0.1, 0.499] */
+  float z_offset;                   /* [0] added to the ray origin's z */
+  int32_t max_point_num_in_cell;    /* [10] >= 1 */
+} sm_mrvm_settings;
+/* Constructor + Initialise (:36-48).  SM_ERR_BAD_ARGUMENT where map_builder_options.cc:66-68 CHECK-fails
+ * (hit_prob <= 0.5, miss_prob >= 0.5, max_point_num_in_cell < 1) and for high_resolution <= 0.  expected_voxels
+ * sizes the first allocation; the map grows past it as needed. */
+int sm_mrvm_create(int device, const sm_mrvm_settings* settings, int64_t expected_voxels, sm_mrvm** out);
+int sm_mrvm_destroy(sm_mrvm* h);
+/* SetOffsetZ (:50-52). */
+int sm_mrvm_set_offset_z(sm_mrvm* h, float offset);
+/* InsertPointCloud (:54-123); origin = the sensor position, 3 floats.  An empty cloud leaves the map unchanged.
+ * Returns the number of points dropped for a non-finite coordinate (>= 0), or an sm_error.  The _device form
+ * reads device memory and orders itself after the work already queued on `cuda_stream` (a cudaStream_t, NULL = the
+ * legacy default stream). */
+int sm_mrvm_insert(sm_mrvm* h, const float* points, int64_t n, int64_t stride_bytes, const float* origin_3);
+int sm_mrvm_insert_device(sm_mrvm* h, const float* dev_points, int64_t n, int64_t stride_bytes,
+                          const float* origin_3, void* cuda_stream);
+/* Number of voxels in the map (high_resolution_voxels_.size()). */
+int64_t sm_mrvm_size(const sm_mrvm* h);
+/* OutputToPointCloud (:125-215): voxels with probability >= (uint8)(threshold * 256) in ascending voxel order.
+ * out4: records {x, y, z, value}; with output_average one record per voxel (the float mean of its stored points,
+ * summed in stored order), otherwise one per stored point.  value: rgb = 0 (the PointXYZI overload):
+ * max_intensity if use_max_intensity, else 0 for a mean and the point's own intensity for a stored point;
+ * rgb = 1 (the PointXYZRGB overload): the grey level min(255, (uint32)(max_intensity * 1.4)).  *m_out = number of
+ * records; SM_ERR_BAD_ARGUMENT if it exceeds `capacity` (out4 untouched) or threshold * 256 is outside (-1, 256). */
+int sm_mrvm_output(sm_mrvm* h, float threshold, int32_t rgb, float* out4, int64_t capacity, int64_t* m_out);
+/* Cumulative device time of the insert phases, from CUDA events: [0] upload, [1] end keys + sort + segments,
+ * [2] table insert (and growth), [3] rays, [4] voxel update; [5] = number of inserts. */
+int sm_mrvm_phase_ms(const sm_mrvm* h, float* ms_6);
+
 int sm_device_count(void);
 const char* sm_version(void);
 

@@ -18,7 +18,10 @@
  *     sm_debug_voxel_index     the voxel index of a point in the submap filter, the NDT grid and ApproximateVoxelGrid
  *     sm_debug_motion_host     InterpolateTransform(Identity, delta, factor) applied to a point
  *     sm_debug_normals_leaf    the leaf plane fit of CalculateNormals (cloud_types.cc:73-103)
+ *     sm_debug_mrvm_ray        the Bresenham ray of one point of MultiResolutionVoxelMap::InsertPointCloud
+ *     sm_debug_mrvm_update     its per-voxel probability update (misses, then hits, by binary lifting)
  *   on the device
+ *     sm_debug_mrvm_state      the full state of a MultiResolutionVoxelMap, for bit-level comparison with the oracle
  *     sm_debug_solve6          the 6x6 solver exactly as icp_finish_kernel calls it
  *     sm_debug_knn1_batched    sm_knn1 with the scheduling the ICP iteration uses when many alignments are in flight
  *                              (queries_per_cta > 256: lockstep root visits, then the lanes of a warp pull parked
@@ -136,6 +139,24 @@ int sm_debug_ndt_leaf(const float* points_3n, int32_t n, int32_t min_points, dou
 int sm_debug_ndt_term(const double* p_6, double outlier_ratio, float resolution, int32_t f64_math,
                       const float* x_orig_3, const float* x_trans_3, const double* voxel_mean_3,
                       const double* voxel_icov_9, double* out43);
+
+/* The ray of one point of MultiResolutionVoxelMap::InsertPointCloud (csrc/mrvm.cu mrvm_voxel + mrvm_walk compiled for
+ * the host, common::VoxelCastingBresenham math.cc:35-95): the voxels from origin's to point's, both included,
+ * 3 int32 each.  *n_out = number of voxels; SM_ERR_BAD_ARGUMENT for a non-finite or out-of-range coordinate, or when
+ * it exceeds `capacity`. */
+int sm_debug_mrvm_ray(const float* origin_3, const float* point_3, float step, int32_t* voxels_3n, int64_t capacity,
+                      int64_t* n_out);
+/* The per-voxel probability update of an insert (csrc/mrvm.cu mrvm_tables + mrvm_lift): probs[i] after misses[i]
+ * misses and then hits[i] hits (each < 2^32), for hit_prob / miss_prob as sm_mrvm_create takes them.  tables_out
+ * (optional, 512 bytes): the one-step hit and miss maps. */
+int sm_debug_mrvm_update(float hit_prob, float miss_prob, const uint8_t* probs, const int64_t* misses,
+                         const int64_t* hits, int64_t n, uint8_t* out, uint8_t* tables_out);
+/* Full state of a map in ascending key order (for bit-level comparison): key = ((ix + 2^20) << 42) |
+ * ((iy + 2^20) << 21) | (iz + 2^20), probability, max_intensity, number of stored points, and the stored points
+ * {x, y, z, intensity} (max_point_num_in_cell records per voxel, unused ones zero).  *n_out = number of voxels;
+ * SM_ERR_BAD_ARGUMENT if it exceeds `capacity`. */
+int sm_debug_mrvm_state(struct sm_mrvm* h, int64_t* keys, uint8_t* prob, int32_t* max_intensity, int32_t* npts,
+                        float* points4, int64_t capacity, int64_t* n_out);
 
 #ifdef __cplusplus
 }

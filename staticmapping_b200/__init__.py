@@ -3,7 +3,7 @@ registrator::Interface.  The compute lives in libsm_b200.so (hand-written sm_100
 C ABI in include/sm_b200.h); this package is the thin host-side mirror used by the tests
 and the bench.  There is no CPU fallback."""
 from .registrators import (AlignBatch, AlignPairs, CalculateNormals, CheckFailure, CreateMatcher, EigenCloud, IcpFast, IcpUsingPointMatcher, InnerCloud,  # noqa: F401
-                           Interface, M2dp, MatcherOptions, matchTwoM2dpDescriptors, MotionCompensation, AverageTransforms, Ndt, NdtWithGicp, Type, VoxelGridFilter, knn1)
+                           Interface, M2dp, MatcherOptions, MrvmSettings, MultiResolutionVoxelMap, matchTwoM2dpDescriptors, MotionCompensation, AverageTransforms, Ndt, NdtWithGicp, Type, VoxelGridFilter, knn1)
 
 __all__ = ["AlignBatch", "AlignPairs", "CalculateNormals", "CheckFailure", "CreateMatcher", "EigenCloud", "IcpFast", "IcpUsingPointMatcher", "InnerCloud", "Interface", "M2dp", "matchTwoM2dpDescriptors", "Ndt", "NdtWithGicp",
-           "MatcherOptions", "MotionCompensation", "AverageTransforms", "Type", "VoxelGridFilter", "knn1"]
+           "MatcherOptions", "MotionCompensation", "MrvmSettings", "MultiResolutionVoxelMap", "AverageTransforms", "Type", "VoxelGridFilter", "knn1"]

@@ -69,6 +69,14 @@ SIGNATURES = {
     "sm_m2dp": (C.c_int, [C.c_int, _VP, C.c_int64, C.c_int64, C.c_double, C.c_double, C.c_int32, C.c_int32, C.c_int32,
                           _VP, C.c_int64, _VP]),
     "sm_m2dp_match": (C.c_double, [_VP, _VP, C.c_int64]),
+    "sm_mrvm_create": (C.c_int, [C.c_int, _VP, C.c_int64, C.POINTER(_VP)]),
+    "sm_mrvm_destroy": (C.c_int, [_VP]),
+    "sm_mrvm_set_offset_z": (C.c_int, [_VP, C.c_float]),
+    "sm_mrvm_insert": (C.c_int, [_VP, _VP, C.c_int64, C.c_int64, _VP]),
+    "sm_mrvm_insert_device": (C.c_int, [_VP, _VP, C.c_int64, C.c_int64, _VP, _VP]),
+    "sm_mrvm_size": (C.c_int64, [_VP]),
+    "sm_mrvm_output": (C.c_int, [_VP, C.c_float, C.c_int32, _VP, C.c_int64, C.POINTER(C.c_int64)]),
+    "sm_mrvm_phase_ms": (C.c_int, [_VP, _VP]),
     # include/sm_b200_debug.h (test hooks)
     "sm_debug_solve6": (C.c_int, [C.c_int, _VP, _VP, _VP, _VP]),
     "sm_debug_solve6_host": (C.c_int, [_VP, _VP, _VP, _VP]),
@@ -85,6 +93,9 @@ SIGNATURES = {
     "sm_debug_ndt_leaf": (C.c_int, [_VP, C.c_int32, C.c_int32, C.c_double, _VP, _VP, _VP, _VP, _VP]),
     "sm_debug_ndt_term": (C.c_int, [_VP, C.c_double, C.c_float, C.c_int32, _VP, _VP, _VP, _VP, _VP]),
     "sm_debug_ndt_host": (C.c_int, [C.c_int32, _VP, _VP]),
+    "sm_debug_mrvm_ray": (C.c_int, [_VP, _VP, C.c_float, _VP, C.c_int64, C.POINTER(C.c_int64)]),
+    "sm_debug_mrvm_update": (C.c_int, [C.c_float, C.c_float, _VP, _VP, _VP, C.c_int64, _VP, _VP]),
+    "sm_debug_mrvm_state": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, C.c_int64, C.POINTER(C.c_int64)]),
     "sm_debug_knn1_batched": (C.c_int, [C.c_int, _VP, C.c_int64, _VP, C.c_int64, C.c_double, C.c_int, C.c_int32, _VP, _VP]),
     "sm_device_count": (C.c_int, []),
     "sm_version": (C.c_char_p, []),

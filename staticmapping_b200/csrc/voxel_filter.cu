@@ -155,6 +155,17 @@ vf_mean_kernel(const float4* __restrict__ sorted, const uint32_t* __restrict__ v
 
 }  // namespace
 
+// segment heads of sorted keys (~0 = dropped point, sorted behind every voxel): starts[v] = first sorted position of
+// segment v, starts[count] = n - meta[3]; block_sum[ceil(n / 2048)] = count.  Also used by mrvm.cu.
+void segment_heads_launch(const uint64_t* keys, int n, uint32_t* block_sum, uint32_t* starts, const long long* meta,
+                          cudaStream_t s) {
+  const int nblk = ceil_div(n, kTile);
+  vf_heads_count_kernel<<<nblk, kT, 0, s>>>(keys, n, block_sum);
+  cudaMemsetAsync(block_sum + nblk, 0, sizeof(uint32_t), s);
+  radix_scan_kernel_launch(block_sum, nblk + 1, 1, s);                                // block_sum[nblk] = number of voxels
+  vf_heads_scatter_kernel<<<nblk, kT, 0, s>>>(keys, n, block_sum, starts, meta);
+}
+
 // host build of the voxel index of one point (test hook sm_debug_voxel_index op 0)
 bool vf_debug_index_host(const float* p, float voxel, long long* ixyz) { return vf_index(p, voxel, &ixyz[0], &ixyz[1], &ixyz[2]); }
 }  // namespace smb
@@ -206,10 +217,7 @@ extern "C" int sm_voxel_grid_filter(int device, const float* points, int64_t n, 
   vf_key_kernel<<<ceil_div(n, 256), 256, 0, s>>>(d_in, stride_bytes, ni, voxel_size, keys0, ord0, meta);
   rc = radix_sort_pairs_u64(keys0, ord0, keys1, ord1, ni, 1, st, scratch, s, 8);   // 8 passes: result back in [0]
   if (rc) return fail(rc == -100 ? SM_ERR_CUDA : rc);
-  vf_heads_count_kernel<<<nblk, kT, 0, s>>>(keys0, ni, block_sum);
-  cudaMemsetAsync(block_sum + nblk, 0, sizeof(uint32_t), s);
-  radix_scan_kernel_launch(block_sum, nblk + 1, 1, s);                                // block_sum[nblk] = number of voxels
-  vf_heads_scatter_kernel<<<nblk, kT, 0, s>>>(keys0, ni, block_sum, voxel_start, meta);
+  segment_heads_launch(keys0, ni, block_sum, voxel_start, meta, s);                   // block_sum[nblk] = number of voxels
   vf_gather_kernel<<<ceil_div(n, 256), 256, 0, s>>>(d_in, stride_bytes, ord0, ni, sorted);
   vf_mean_kernel<<<ceil_div((int64_t)n * 32, 256), 256, 0, s>>>(sorted, voxel_start, block_sum + nblk, d_out);
   uint32_t m = 0;

@@ -578,3 +578,124 @@ def matchTwoM2dpDescriptors(P, Q):
     if P.shape != Q.shape:
         return -1.0
     return float(_lib.lib().sm_m2dp_match(P.ctypes.data, Q.ctypes.data, P.shape[0]))
+
+
+class MrvmSettings(C.Structure):
+    """MrvmSettings (builder/multi_resolution_voxel_map.h:55-66) == sm_mrvm_settings; the reference's defaults."""
+    _fields_ = [("output_average", C.c_int32), ("output_rgb", C.c_int32), ("use_max_intensity", C.c_int32),
+                ("prob_threshold", C.c_float), ("low_resolution", C.c_float), ("high_resolution", C.c_float),
+                ("hit_prob", C.c_float), ("miss_prob", C.c_float), ("z_offset", C.c_float),
+                ("max_point_num_in_cell", C.c_int32)]
+
+    def __init__(self, output_average=False, output_rgb=False, use_max_intensity=True, prob_threshold=0.6,
+                 low_resolution=1.0, high_resolution=0.1, hit_prob=0.55, miss_prob=0.48, z_offset=0.0,
+                 max_point_num_in_cell=10):
+        super().__init__(int(output_average), int(output_rgb), int(use_max_intensity), prob_threshold, low_resolution,
+                         high_resolution, hit_prob, miss_prob, z_offset, int(max_point_num_in_cell))
+
+
+class MultiResolutionVoxelMap:
+    """builder::MultiResolutionVoxelMap (multi_resolution_voxel_map.{h,cc}) on the GPU: the ray-casting occupancy
+    map that removes moving objects from static_map.pcd.  The map stays on the device between inserts.  Semantics:
+    the reference's run by one thread; voxels are output in ascending (ix, iy, iz) order (include/sm_b200.h)."""
+
+    def __init__(self, device=0, expected_voxels=1 << 20):
+        self.device, self.expected_voxels = device, int(expected_voxels)
+        self.settings = None
+        self._h = None
+
+    def __del__(self):
+        self._release()
+
+    def _release(self):
+        if getattr(self, "_h", None):
+            _lib.lib().sm_mrvm_destroy(self._h)
+            self._h = None
+
+    def _check(self, rc, what):
+        if rc == -20:
+            raise RuntimeError("staticmapping_b200: no CUDA device (no CPU fallback)")
+        if rc == -1:
+            raise CheckFailure(f"MultiResolutionVoxelMap::{what}: invalid argument")
+        if rc < 0:
+            raise RuntimeError(f"MultiResolutionVoxelMap::{what} failed with {rc}")
+        return rc
+
+    def Initialise(self, settings: MrvmSettings):
+        """Initialise (:42-48) on an empty map.  CheckFailure where map_builder_options.cc:66-68 CHECK-fails
+        (hit_prob <= 0.5, miss_prob >= 0.5, max_point_num_in_cell < 1) or high_resolution <= 0."""
+        self._release()
+        h = C.c_void_p()
+        self._check(_lib.lib().sm_mrvm_create(self.device, C.byref(settings), self.expected_voxels, C.byref(h)),
+                    "Initialise")
+        self._h, self.settings = h, settings
+
+    def SetOffsetZ(self, offset):
+        self._check(_lib.lib().sm_mrvm_set_offset_z(self._handle(), float(offset)), "SetOffsetZ")
+
+    def _handle(self):
+        if not self._h:
+            raise CheckFailure("MultiResolutionVoxelMap: Initialise first")
+        return self._h
+
+    def InsertPointCloud(self, cloud, origin):
+        """cloud: (N,5) float32 InnerPointType rows (x, y, z, intensity, factor) as a numpy array, or a C-contiguous
+        float32 CUDA tensor of the same shape (read in place, after the work queued on torch's current stream).
+        origin: sensor position (3,).  Returns the number of points dropped for a non-finite coordinate; raises
+        CheckFailure (map unchanged) for a voxel index outside [-2^20, 2^20)."""
+        o = np.ascontiguousarray(np.asarray(origin, dtype=np.float32).reshape(3))
+        lib = _lib.lib()
+        if hasattr(cloud, "is_cuda") and cloud.is_cuda:
+            import torch
+            if cloud.dtype != torch.float32 or cloud.dim() != 2 or cloud.shape[1] != 5 or not cloud.is_contiguous():
+                raise ValueError("cloud must be a contiguous (N,5) float32 tensor")
+            stream = torch.cuda.current_stream(cloud.device).cuda_stream
+            rc = lib.sm_mrvm_insert_device(self._handle(), cloud.data_ptr(), cloud.shape[0], 20, o.ctypes.data, stream)
+        else:
+            pts = np.ascontiguousarray(np.asarray(cloud, dtype=np.float32))
+            if pts.ndim != 2 or pts.shape[1] != 5:
+                raise ValueError("cloud must be (N,5): x, y, z, intensity, factor")
+            rc = lib.sm_mrvm_insert(self._handle(), pts.ctypes.data, pts.shape[0], 20, o.ctypes.data)
+        return self._check(rc, "InsertPointCloud")
+
+    def size(self):
+        return int(_lib.lib().sm_mrvm_size(self._handle()))
+
+    def OutputToPointCloud(self, threshold=None, rgb=None):
+        """OutputToPointCloud (:125-215) -> (M,4) float32 {x, y, z, value}.  threshold defaults to
+        settings.prob_threshold, rgb to settings.output_rgb; value is the intensity (PointXYZI) or the grey level
+        (PointXYZRGB)."""
+        h = self._handle()
+        t = float(self.settings.prob_threshold if threshold is None else threshold)
+        r = int(bool(self.settings.output_rgb if rgb is None else rgb))
+        lib = _lib.lib()
+        m = C.c_int64(0)
+        rc = lib.sm_mrvm_output(h, t, r, None, 0, C.byref(m))
+        if rc == -1 and m.value > 0:
+            out = np.empty((m.value, 4), np.float32)
+            rc = lib.sm_mrvm_output(h, t, r, out.ctypes.data, m.value, C.byref(m))
+            self._check(rc, "OutputToPointCloud")
+            return out
+        self._check(rc, "OutputToPointCloud")
+        return np.zeros((0, 4), np.float32)
+
+    def PhaseMs(self):
+        """Cumulative device time of the insert phases (CUDA events): upload, keys + sort + segments, table insert,
+        rays, voxel update; and the number of inserts."""
+        ms = np.zeros(6, np.float32)
+        self._check(_lib.lib().sm_mrvm_phase_ms(self._handle(), ms.ctypes.data), "PhaseMs")
+        return {"upload": float(ms[0]), "keys_sort_segments": float(ms[1]), "table_insert": float(ms[2]),
+                "rays": float(ms[3]), "update": float(ms[4]), "inserts": int(ms[5])}
+
+    def State(self):
+        """Test hook sm_debug_mrvm_state: dict(keys, prob, max_intensity, npts, points (n, max_point_num_in_cell, 4))
+        in ascending key order."""
+        h = self._handle()
+        n = self.size()
+        mp = self.settings.max_point_num_in_cell
+        keys = np.zeros(n, np.int64); prob = np.zeros(n, np.uint8)
+        mi = np.zeros(n, np.int32); npts = np.zeros(n, np.int32); pts = np.zeros((n, mp, 4), np.float32)
+        got = C.c_int64(0)
+        self._check(_lib.lib().sm_debug_mrvm_state(h, keys.ctypes.data, prob.ctypes.data, mi.ctypes.data,
+                                                   npts.ctypes.data, pts.ctypes.data, n, C.byref(got)), "State")
+        return {"keys": keys, "prob": prob, "max_intensity": mi, "npts": npts, "points": pts}
