@@ -333,6 +333,49 @@ class MultiResolutionVoxelMapB200 {
   sm_mrvm* handle_ = nullptr;
 };
 
+// pre_processers::filter::Factory (pre_processors/filter_factory.cc:63-123) on the GPU.  Stages come in XML order as
+// (filter name, [(param name, type attribute, text)]); Filter runs them on a data::InnerCloudType.  Semantics and
+// deviations: include/sm_b200.h (sm_filter_chain_*).
+class FilterFactoryB200 {
+ public:
+  struct Param { std::string name; int type; std::string text; };
+  explicit FilterFactoryB200(int device = 0, uint64_t seed = 0) {
+    const int rc = sm_filter_chain_create(device, &handle_);
+    CHECK_EQ(rc, 0) << "sm_filter_chain_create failed (" << rc << "): no CUDA device";
+    sm_filter_chain_set_seed(handle_, seed);
+  }
+  ~FilterFactoryB200() { if (handle_) sm_filter_chain_destroy(handle_); }
+  FilterFactoryB200(const FilterFactoryB200&) = delete;
+  FilterFactoryB200& operator=(const FilterFactoryB200&) = delete;
+
+  // Factory::InitFromXmlNode for one <filter>: an unknown name or parameter is a CHECK failure here
+  void AddFilter(const std::string& name, const std::vector<Param>& params) {
+    const int stage = sm_filter_chain_add(handle_, name.c_str());
+    CHECK_GE(stage, 0) << name << " not supported";
+    for (const Param& p : params)
+      CHECK_EQ(sm_filter_chain_set_param(handle_, stage, p.name.c_str(), p.type, p.text.c_str()), 0)
+          << name << ": cannot set " << p.name;
+  }
+
+  // Factory::Filter: `cloud` (a data::InnerCloudType::Ptr, or any pointer to one) in, the filtered cloud out
+  template <typename CloudPtr>
+  void Filter(const CloudPtr& cloud) {
+    CHECK(cloud);
+    const int64_t n = static_cast<int64_t>(cloud->points.size());
+    if (n == 0) return;
+    std::vector<data::InnerPointType> out(static_cast<size_t>(n));
+    int64_t m = 0;
+    const int rc = sm_filter_chain_filter(handle_, &cloud->points[0].x, n, sizeof(data::InnerPointType), &out[0].x, n,
+                                          &m, nullptr);
+    CHECK_EQ(rc, 0) << "sm_filter_chain_filter failed (" << rc << "): invalid stage or CUDA failure";
+    out.resize(static_cast<size_t>(m));
+    cloud->points.assign(out.begin(), out.end());
+  }
+
+ private:
+  sm_filter_chain* handle_ = nullptr;
+};
+
 }  // namespace registrator
 }  // namespace static_map
 

@@ -321,6 +321,72 @@ int sm_mrvm_output(sm_mrvm* h, float threshold, int32_t rgb, float* out4, int64_
  * [2] table insert (and growth), [3] rays, [4] voxel update; [5] = number of inserts. */
 int sm_mrvm_phase_ms(const sm_mrvm* h, float* ms_6);
 
+/* pre_processers::filter::Factory (pre_processors/filter_factory.cc:63-123) and its nine filters, the <filters> chain
+ * DataCollector::CloudPreProcessing runs on every scan (builder/data/data_collector.cc:120-156).  A handle holds the
+ * stages in XML order; sm_filter_chain_add takes the filter's name (RandomSampler, RangeImage, GroundRemoval,
+ * GroundRemoval2, Range, StatisticRemoval, VoxelGrid, AxisRange, BoundingBoxRemoval) and returns the stage index,
+ * SM_ERR_UNSUPPORTED_TYPE for any other name (the reference skips it with a log line).  sm_filter_chain_set_param is
+ * one <param type=... name=...>text</param>: type 0 parses text like pugixml's as_int, type 1 like as_float, and the
+ * value is cast to the parameter's own type; SM_ERR_UNKNOWN_OPTION for a name the filter does not register (a CHECK
+ * failure in the reference), SM_ERR_BAD_ARGUMENT for another type.  Parameters keep their values until set again.
+ * sm_filter_chain_valid: the filter's ConfigsValid() (1 / 0).
+ * Points are data::InnerPointType records {x, y, z, intensity, factor} `stride_bytes` (>= 20) apart; `out` receives
+ * records of 5 packed floats, `kept_index` (optional) the chain-input index of each output record (-1 behind a
+ * VoxelGrid).  *m_out = number of output records; SM_ERR_BAD_ARGUMENT if it exceeds `capacity` (out untouched).
+ * Every filter keeps the reference's semantics, quirks included:
+ *   Range: r = sqrtf(x*x + y*y + z*z), kept iff min_range <= r <= max_range (a NaN point is removed).
+ *   AxisRange: removed iff v < min || v > max on axis_index; the identity at min = -FLT_MAX and max = FLT_MAX, and for
+ *     an axis_index outside 0..2; a NaN coordinate is kept.
+ *   BoundingBoxRemoval: removes the points inside the box, bounds included (the default box removes every finite point).
+ *   RangeImage: the first point in input order that lands in a pixel is kept; rows truncate toward zero (a point up to
+ *     one row below btm_angle lands in row 0), columns are lround of a float quotient wrapped once; xy < 0.01 and a
+ *     row or column outside the image are outliers.
+ *   GroundRemoval: voxels static_cast<int>(v / leaf_size); voxels with fewer than min_point_num_in_voxel points vanish;
+ *     a voxel with iz <= 0 and max z - min z <= height_threshold is ground.  Output in std::map order: ascending
+ *     (ix, iy, iz), input order inside a voxel.
+ *   GroundRemoval2: the reference's binning, FitLines and ClusterGround, serially per segment.
+ *   VoxelGrid: sm_voxel_grid_filter.
+ * Deviations from the reference:
+ *   1. RandomSampler seeds std::mt19937 from std::random_device on every call, so its result is not a function of its
+ *      inputs.  Here a point is kept iff u <= sampling_rate, u uniform on [0, 1) from a counter hash of (seed, call
+ *      number, stage index, chain-input index); the call number starts at 0 at sm_filter_chain_set_seed and advances
+ *      once per filter call.  A rate above 0.999 is the identity, as in the reference.
+ *   2. Angles (RangeImage's pixel, GroundRemoval2's segment) use one atan2: a double-precision evaluation from
+ *      correctly rounded +, -, *, / and sqrt, rounded to float, the same bits on the host and the device.  libm's
+ *      atan2f is not the same function on every C library (glibc's differs from (float)atan2((double)y, x) on about
+ *      16 % of random points), so pixel and cell indices equal a reference run's only given the same angle function.
+ *   3. GroundRemoval2's line fit is a two-column Householder QR with column pivoting in double; Eigen's
+ *      colPivHouseholderQr rounds through vectorised reductions, so m and b agree to float rounding, not bit for bit.
+ *   4. StatisticRemoval (its body is commented out in the reference) is the identity.  As the FIRST stage the
+ *      reference's Factory returns an empty cloud (the untouched intermediate cloud); that bug is not reproduced.
+ *   5. A stage whose ConfigsValid() is false, or that this engine cannot run (RangeImage with a line count <= 0,
+ *      GroundRemoval with leaf_size 0, GroundRemoval2 with bin_num or segment_num <= 0 or a search angle of a full
+ *      turn), makes the call return SM_ERR_BAD_ARGUMENT without output; the reference runs it anyway (or divides by 0).
+ *   6. Non-finite points: RangeImage drops a point whose row is NaN; GroundRemoval and GroundRemoval2 do not bin them:
+ *      they stay inliers (GroundRemoval emits them after every voxel) and are never ground.  GroundRemoval returns
+ *      SM_ERR_BAD_ARGUMENT for a voxel index outside the int range or finite points spanning 2^21 voxels on one axis.
+ *   7. thread_num of GroundRemoval2 is accepted and ignored.
+ * The _device form takes device pointers (in, out and kept_index), orders itself after the work queued on
+ * `cuda_stream` and reads back only the count.  Every call returns after its device work has finished.  One handle is
+ * used by one thread at a time; it owns its CUDA stream. */
+typedef struct sm_filter_chain sm_filter_chain;
+int sm_filter_chain_create(int device, sm_filter_chain** out);
+int sm_filter_chain_destroy(sm_filter_chain* h);
+int sm_filter_chain_add(sm_filter_chain* h, const char* name);
+int sm_filter_chain_set_param(sm_filter_chain* h, int32_t stage, const char* name, int32_t type, const char* text);
+int sm_filter_chain_valid(const sm_filter_chain* h, int32_t stage);
+int sm_filter_chain_set_seed(sm_filter_chain* h, uint64_t seed);
+int sm_filter_chain_filter(sm_filter_chain* h, const float* points, int64_t n, int64_t stride_bytes, float* out,
+                           int64_t capacity, int64_t* m_out, int32_t* kept_index);
+int sm_filter_chain_filter_device(sm_filter_chain* h, const float* dev_points, int64_t n, int64_t stride_bytes,
+                                  float* dev_out, int64_t capacity, int64_t* m_out, int32_t* dev_kept_index,
+                                  void* cuda_stream);
+/* Points after each stage of the last call (counts[k] for k < n); returns the number of stages. */
+int sm_filter_chain_stage_counts(const sm_filter_chain* h, int64_t* counts, int32_t n);
+/* Device time of each stage of the last call, from CUDA events (a fused run of point-wise stages is reported on its
+ * first stage, the initial gather on the first step); returns the number of stages. */
+int sm_filter_chain_stage_ms(const sm_filter_chain* h, float* ms, int32_t n);
+
 int sm_device_count(void);
 const char* sm_version(void);
 

@@ -158,6 +158,23 @@ int sm_debug_mrvm_update(float hit_prob, float miss_prob, const uint8_t* probs, 
 int sm_debug_mrvm_state(struct sm_mrvm* h, int64_t* keys, uint8_t* prob, int32_t* max_intensity, int32_t* npts,
                         float* points4, int64_t capacity, int64_t* n_out);
 
+/* The per-point functions of the filter chain (csrc/filters.cu), compiled for the host, over n points `stride_bytes`
+ * apart:
+ *   op 0: the product's atan2f(y, x), out[k] = its float bits                       params unused
+ *   op 1: RangeImage pixel row * H + col, -1 outlier      params = top, btm, offset_x, offset_y, offset_z, V, H
+ *   op 2: GroundRemoval2 cell s * bin_num + b, -1 not binned   params = r_max, r_min, bin_num, segment_num
+ *   op 3: GroundRemoval voxel, out[4k..4k+3] = rc (0 ok, 1 not finite, 2 outside int), ix, iy, iz   params = leaf */
+int sm_debug_filter_points(int32_t op, const float* points, int64_t n, int64_t stride_bytes, const float* params,
+                           int64_t* out);
+/* GroundRemoval2::FitLines of one segment: cell_dz = bin_num (d, z) min_z_points, cell_used = bin_num flags (the
+ * cell's `points` is not empty); params = r_max, r_min, start_ground_height, long_line_threshold, max_long_line_height,
+ * max_start_height, max_error, max_slope, max_b, max_dist_to_line, search_angle, bin_num.  lines4: (start d, start z,
+ * end d, end z) per line; *n_out = number of lines. */
+int sm_debug_filter_fit_lines(const float* cell_dz, const uint8_t* cell_used, const float* params, float* lines4,
+                              int64_t capacity, int64_t* n_out);
+/* FitLocalLine + GetMaxError over k (d, z) points: mb = m, b, max error. */
+int sm_debug_filter_line_fit(const float* dz, int64_t k, float* mb);
+
 #ifdef __cplusplus
 }
 #endif

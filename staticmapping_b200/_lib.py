@@ -77,6 +77,17 @@ SIGNATURES = {
     "sm_mrvm_size": (C.c_int64, [_VP]),
     "sm_mrvm_output": (C.c_int, [_VP, C.c_float, C.c_int32, _VP, C.c_int64, C.POINTER(C.c_int64)]),
     "sm_mrvm_phase_ms": (C.c_int, [_VP, _VP]),
+    "sm_filter_chain_create": (C.c_int, [C.c_int, C.POINTER(_VP)]),
+    "sm_filter_chain_destroy": (C.c_int, [_VP]),
+    "sm_filter_chain_add": (C.c_int, [_VP, C.c_char_p]),
+    "sm_filter_chain_set_param": (C.c_int, [_VP, C.c_int32, C.c_char_p, C.c_int32, C.c_char_p]),
+    "sm_filter_chain_valid": (C.c_int, [_VP, C.c_int32]),
+    "sm_filter_chain_set_seed": (C.c_int, [_VP, C.c_uint64]),
+    "sm_filter_chain_filter": (C.c_int, [_VP, _VP, C.c_int64, C.c_int64, _VP, C.c_int64, C.POINTER(C.c_int64), _VP]),
+    "sm_filter_chain_filter_device": (C.c_int, [_VP, _VP, C.c_int64, C.c_int64, _VP, C.c_int64, C.POINTER(C.c_int64),
+                                                _VP, _VP]),
+    "sm_filter_chain_stage_counts": (C.c_int, [_VP, _VP, C.c_int32]),
+    "sm_filter_chain_stage_ms": (C.c_int, [_VP, _VP, C.c_int32]),
     # include/sm_b200_debug.h (test hooks)
     "sm_debug_solve6": (C.c_int, [C.c_int, _VP, _VP, _VP, _VP]),
     "sm_debug_solve6_host": (C.c_int, [_VP, _VP, _VP, _VP]),
@@ -96,6 +107,9 @@ SIGNATURES = {
     "sm_debug_mrvm_ray": (C.c_int, [_VP, _VP, C.c_float, _VP, C.c_int64, C.POINTER(C.c_int64)]),
     "sm_debug_mrvm_update": (C.c_int, [C.c_float, C.c_float, _VP, _VP, _VP, C.c_int64, _VP, _VP]),
     "sm_debug_mrvm_state": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, C.c_int64, C.POINTER(C.c_int64)]),
+    "sm_debug_filter_points": (C.c_int, [C.c_int32, _VP, C.c_int64, C.c_int64, _VP, _VP]),
+    "sm_debug_filter_fit_lines": (C.c_int, [_VP, _VP, _VP, _VP, C.c_int64, C.POINTER(C.c_int64)]),
+    "sm_debug_filter_line_fit": (C.c_int, [_VP, C.c_int64, _VP]),
     "sm_debug_knn1_batched": (C.c_int, [C.c_int, _VP, C.c_int64, _VP, C.c_int64, C.c_double, C.c_int, C.c_int32, _VP, _VP]),
     "sm_device_count": (C.c_int, []),
     "sm_version": (C.c_char_p, []),

@@ -225,6 +225,9 @@ struct GicpCostParams {     // one BFGS function evaluation (:255-377)
 // voxel_filter.cu: segment heads of radix-sorted keys (~0 = dropped, meta[3] of them), shared with mrvm.cu
 void segment_heads_launch(const uint64_t* keys, int n, uint32_t* block_sum, uint32_t* starts, const long long* meta,
                           cudaStream_t s);
+// VoxelGrid::Filter of a device cloud into d_out (capacity n records of 5 floats); shared with filters.cu
+int voxel_grid_device(const char* d_in, int64_t stride, int n, float voxel_size, float* d_out, uint32_t* m_out,
+                      cudaStream_t s);
 // host builds of the three voxel-index functions (test hook sm_debug_voxel_index)
 bool vf_debug_index_host(const float* p, float voxel, long long* ixyz);
 int ndt_debug_voxel_coord_host(float v, float inv_leaf, int min_b);

@@ -168,6 +168,56 @@ void segment_heads_launch(const uint64_t* keys, int n, uint32_t* block_sum, uint
 
 // host build of the voxel index of one point (test hook sm_debug_voxel_index op 0)
 bool vf_debug_index_host(const float* p, float voxel, long long* ixyz) { return vf_index(p, voxel, &ixyz[0], &ixyz[1], &ixyz[2]); }
+// VoxelGrid::Filter over a device cloud (records `stride` >= 16 bytes apart): d_out receives *m_out records of 5 floats
+// (capacity n), in ascending voxel order.  Returns after the stream has finished.  Also used by filters.cu.
+int voxel_grid_device(const char* d_in, int64_t stride, int n, float voxel_size, float* d_out, uint32_t* m_out,
+                      cudaStream_t s) {
+  *m_out = 0;
+  if (n == 0) return SM_OK;
+  const int ni = n;
+  const int nblk = ceil_div(n, kTile);
+  const int64_t st = ((int64_t)n + 63) & ~(int64_t)63;
+  size_t bytes = 256;
+  bytes += 2 * st * sizeof(uint64_t) + 2 * st * sizeof(uint32_t);            // keys, order (ping-pong)
+  bytes += radix_sort_scratch_bytes(ni, 1) + 256;
+  bytes += ((size_t)nblk + 8) * sizeof(uint32_t) + ((size_t)n + 8) * sizeof(uint32_t);   // block sums, voxel_start
+  bytes += (size_t)n * sizeof(float4) + 1024;
+  char* base = nullptr;
+  if (cudaMalloc(&base, bytes) != cudaSuccess) return SM_ERR_CUDA;
+  char* cur = base;
+  auto take = [&](size_t b) { char* p = cur; cur += (b + 255) & ~(size_t)255; return p; };
+  uint64_t* keys0 = (uint64_t*)take(st * sizeof(uint64_t));
+  uint64_t* keys1 = (uint64_t*)take(st * sizeof(uint64_t));
+  uint32_t* ord0 = (uint32_t*)take(st * sizeof(uint32_t));
+  uint32_t* ord1 = (uint32_t*)take(st * sizeof(uint32_t));
+  uint32_t* scratch = (uint32_t*)take(radix_sort_scratch_bytes(ni, 1));
+  uint32_t* block_sum = (uint32_t*)take(((size_t)nblk + 8) * sizeof(uint32_t));
+  uint32_t* voxel_start = (uint32_t*)take(((size_t)n + 8) * sizeof(uint32_t));
+  float4* sorted = (float4*)take((size_t)n * sizeof(float4));
+  long long* meta = (long long*)take(256);
+  int rc = SM_OK;
+  auto fail = [&](int code) { cudaFree(base); return code; };
+  const long long meta_init[8] = {LLONG_MAX, LLONG_MAX, LLONG_MAX, 0, 0, 0, 0, 0};
+  if (cudaMemcpyAsync(meta, meta_init, sizeof(meta_init), cudaMemcpyHostToDevice, s) != cudaSuccess)
+    return fail(SM_ERR_CUDA);
+  vf_min_kernel<<<ceil_div(n, 256), 256, 0, s>>>(d_in, stride, ni, voxel_size, meta);
+  vf_key_kernel<<<ceil_div(n, 256), 256, 0, s>>>(d_in, stride, ni, voxel_size, keys0, ord0, meta);
+  rc = radix_sort_pairs_u64(keys0, ord0, keys1, ord1, ni, 1, st, scratch, s, 8);   // 8 passes: result back in [0]
+  if (rc) return fail(rc == -100 ? SM_ERR_CUDA : rc);
+  segment_heads_launch(keys0, ni, block_sum, voxel_start, meta, s);                   // block_sum[nblk] = number of voxels
+  vf_gather_kernel<<<ceil_div(n, 256), 256, 0, s>>>(d_in, stride, ord0, ni, sorted);
+  vf_mean_kernel<<<ceil_div((int64_t)n * 32, 256), 256, 0, s>>>(sorted, voxel_start, block_sum + nblk, d_out);
+  uint32_t m = 0;
+  long long host_meta[8] = {0};
+  if (cudaGetLastError() != cudaSuccess ||
+      cudaMemcpyAsync(&m, block_sum + nblk, sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+      cudaMemcpyAsync(host_meta, meta, sizeof(host_meta), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+      cudaStreamSynchronize(s) != cudaSuccess)
+    return fail(SM_ERR_CUDA);
+  if (host_meta[4]) return fail(SM_ERR_BAD_ARGUMENT);   // the finite points span 2^21 voxels or more along an axis
+  *m_out = m;
+  return fail(SM_OK);
+}
 }  // namespace smb
 
 using namespace smb;
@@ -182,55 +232,19 @@ extern "C" int sm_voxel_grid_filter(int device, const float* points, int64_t n, 
   SMB_CUDA_OK(cudaSetDevice(device));
   *m_out = 0;
   if (n == 0) return SM_OK;
-  const int ni = (int)n;
-  const int nblk = ceil_div(n, kTile);
-  const int64_t st = (n + 63) & ~(int64_t)63;
   const size_t in_bytes = (size_t)n * (size_t)stride_bytes;
-  size_t bytes = in_bytes + 256;
-  bytes += 2 * st * sizeof(uint64_t) + 2 * st * sizeof(uint32_t);            // keys, order (ping-pong)
-  bytes += radix_sort_scratch_bytes(ni, 1) + 256;
-  bytes += ((size_t)nblk + 8) * sizeof(uint32_t) + ((size_t)n + 8) * sizeof(uint32_t);   // block sums, voxel_start
-  bytes += (size_t)n * sizeof(float4) + (size_t)n * 5 * sizeof(float) + 1024;
-  char* base = nullptr;
-  if (cudaMalloc(&base, bytes) != cudaSuccess) return SM_ERR_CUDA;
-  char* cur = base;
-  auto take = [&](size_t b) { char* p = cur; cur += (b + 255) & ~(size_t)255; return p; };
-  char* d_in = take(in_bytes);
-  uint64_t* keys0 = (uint64_t*)take(st * sizeof(uint64_t));
-  uint64_t* keys1 = (uint64_t*)take(st * sizeof(uint64_t));
-  uint32_t* ord0 = (uint32_t*)take(st * sizeof(uint32_t));
-  uint32_t* ord1 = (uint32_t*)take(st * sizeof(uint32_t));
-  uint32_t* scratch = (uint32_t*)take(radix_sort_scratch_bytes(ni, 1));
-  uint32_t* block_sum = (uint32_t*)take(((size_t)nblk + 8) * sizeof(uint32_t));
-  uint32_t* voxel_start = (uint32_t*)take(((size_t)n + 8) * sizeof(uint32_t));
-  float4* sorted = (float4*)take((size_t)n * sizeof(float4));
-  float* d_out = (float*)take((size_t)n * 5 * sizeof(float));
-  long long* meta = (long long*)take(256);
+  char* d_in = nullptr;
+  float* d_out = nullptr;
+  auto fail = [&](int code) { cudaFree(d_in); cudaFree(d_out); return code; };
   cudaStream_t s = nullptr;
-  int rc = SM_OK;
-  auto fail = [&](int code) { cudaFree(base); return code; };
-  const long long meta_init[8] = {LLONG_MAX, LLONG_MAX, LLONG_MAX, 0, 0, 0, 0, 0};
-  if (cudaMemcpyAsync(d_in, points, in_bytes, cudaMemcpyHostToDevice, s) != cudaSuccess ||
-      cudaMemcpyAsync(meta, meta_init, sizeof(meta_init), cudaMemcpyHostToDevice, s) != cudaSuccess)
+  if (cudaMalloc(&d_in, in_bytes) != cudaSuccess || cudaMalloc(&d_out, (size_t)n * 5 * sizeof(float)) != cudaSuccess ||
+      cudaMemcpyAsync(d_in, points, in_bytes, cudaMemcpyHostToDevice, s) != cudaSuccess)
     return fail(SM_ERR_CUDA);
-  vf_min_kernel<<<ceil_div(n, 256), 256, 0, s>>>(d_in, stride_bytes, ni, voxel_size, meta);
-  vf_key_kernel<<<ceil_div(n, 256), 256, 0, s>>>(d_in, stride_bytes, ni, voxel_size, keys0, ord0, meta);
-  rc = radix_sort_pairs_u64(keys0, ord0, keys1, ord1, ni, 1, st, scratch, s, 8);   // 8 passes: result back in [0]
-  if (rc) return fail(rc == -100 ? SM_ERR_CUDA : rc);
-  segment_heads_launch(keys0, ni, block_sum, voxel_start, meta, s);                   // block_sum[nblk] = number of voxels
-  vf_gather_kernel<<<ceil_div(n, 256), 256, 0, s>>>(d_in, stride_bytes, ord0, ni, sorted);
-  vf_mean_kernel<<<ceil_div((int64_t)n * 32, 256), 256, 0, s>>>(sorted, voxel_start, block_sum + nblk, d_out);
   uint32_t m = 0;
-  long long host_meta[8] = {0};
-  if (cudaGetLastError() != cudaSuccess ||
-      cudaMemcpyAsync(&m, block_sum + nblk, sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-      cudaMemcpyAsync(host_meta, meta, sizeof(host_meta), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-      cudaStreamSynchronize(s) != cudaSuccess)
-    return fail(SM_ERR_CUDA);
-  if (host_meta[4]) return fail(SM_ERR_BAD_ARGUMENT);   // the finite points span 2^21 voxels or more along an axis
+  const int rc = voxel_grid_device(d_in, stride_bytes, (int)n, voxel_size, d_out, &m, s);
+  if (rc) return fail(rc);
   if (m > 0 && cudaMemcpy(out, d_out, (size_t)m * 5 * sizeof(float), cudaMemcpyDeviceToHost) != cudaSuccess)
     return fail(SM_ERR_CUDA);
   *m_out = (int64_t)m;
-  cudaFree(base);
-  return SM_OK;
+  return fail(SM_OK);
 }

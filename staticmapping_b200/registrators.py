@@ -699,3 +699,285 @@ class MultiResolutionVoxelMap:
         self._check(_lib.lib().sm_debug_mrvm_state(h, keys.ctypes.data, prob.ctypes.data, mi.ctypes.data,
                                                    npts.ctypes.data, pts.ctypes.data, n, C.byref(got)), "State")
         return {"keys": keys, "prob": prob, "max_intensity": mi, "npts": npts, "points": pts}
+
+
+class FilterChain:
+    """sm_filter_chain_* (include/sm_b200.h): the stages of a pre_processers::filter::Factory on the GPU.  Thin: the
+    Python filter classes below drive it, or any object with the same methods (the tests' serial oracle)."""
+
+    def __init__(self, device=0):
+        self.device = device
+        h = C.c_void_p()
+        rc = _lib.lib().sm_filter_chain_create(device, C.byref(h))
+        if rc == -20:
+            raise RuntimeError("staticmapping_b200: no CUDA device (no CPU fallback)")
+        if rc < 0:
+            raise RuntimeError(f"sm_filter_chain_create failed with {rc}")
+        self._h = h
+
+    def __del__(self):
+        if getattr(self, "_h", None):
+            _lib.lib().sm_filter_chain_destroy(self._h)
+            self._h = None
+
+    def add(self, name):
+        return _lib.lib().sm_filter_chain_add(self._h, name.encode())
+
+    def set_param(self, stage, name, type_, text):
+        return _lib.lib().sm_filter_chain_set_param(self._h, stage, name.encode(), type_, text.encode())
+
+    def valid(self, stage):
+        return _lib.lib().sm_filter_chain_valid(self._h, stage)
+
+    def set_seed(self, seed):
+        return _lib.lib().sm_filter_chain_set_seed(self._h, int(seed) & ((1 << 64) - 1))
+
+    def filter(self, points5):
+        """(N,5) float32 -> (rc, (M,5) float32 records, (M,) int32 chain-input indices)."""
+        p = np.ascontiguousarray(points5, np.float32)
+        n = p.shape[0]
+        out = np.empty((max(n, 1), 5), np.float32)
+        kept = np.empty(max(n, 1), np.int32)
+        m = C.c_int64(0)
+        rc = _lib.lib().sm_filter_chain_filter(self._h, p.ctypes.data, n, 20, out.ctypes.data, n, C.byref(m),
+                                               kept.ctypes.data)
+        if rc == -1 and m.value > n:                   # VoxelGrid never grows a cloud; kept for completeness
+            out = np.empty((m.value, 5), np.float32); kept = np.empty(m.value, np.int32)
+            rc = _lib.lib().sm_filter_chain_filter(self._h, p.ctypes.data, n, 20, out.ctypes.data, m.value,
+                                                   C.byref(m), kept.ctypes.data)
+        return rc, out[:m.value].copy(), kept[:m.value].copy()
+
+    def filter_device(self, cloud):
+        """contiguous (N,5) float32 CUDA tensor -> (rc, (M,5) tensor, (M,) int32 tensor), on torch's current stream."""
+        import torch
+        if cloud.dtype != torch.float32 or cloud.dim() != 2 or cloud.shape[1] != 5 or not cloud.is_contiguous():
+            raise ValueError("cloud must be a contiguous (N,5) float32 tensor")
+        n = cloud.shape[0]
+        out = torch.empty((max(n, 1), 5), dtype=torch.float32, device=cloud.device)
+        kept = torch.empty(max(n, 1), dtype=torch.int32, device=cloud.device)
+        m = C.c_int64(0)
+        stream = torch.cuda.current_stream(cloud.device).cuda_stream
+        rc = _lib.lib().sm_filter_chain_filter_device(self._h, cloud.data_ptr(), n, 20, out.data_ptr(), n,
+                                                      C.byref(m), kept.data_ptr(), stream)
+        return rc, out[:m.value], kept[:m.value]
+
+    def stage_counts(self):
+        ns = _lib.lib().sm_filter_chain_stage_counts(self._h, None, 0)
+        c = np.zeros(max(ns, 1), np.int64)
+        _lib.lib().sm_filter_chain_stage_counts(self._h, c.ctypes.data, ns)
+        return c[:ns]
+
+    def stage_ms(self):
+        ns = _lib.lib().sm_filter_chain_stage_ms(self._h, None, 0)
+        c = np.zeros(max(ns, 1), np.float32)
+        _lib.lib().sm_filter_chain_stage_ms(self._h, c.ctypes.data, ns)
+        return c[:ns]
+
+
+def _records(cloud):
+    """InnerCloud / (N,3) / (N,5) -> (N,5) float32 InnerPointType rows (intensity and factor 0 for xyz input)."""
+    p = cloud.points if isinstance(cloud, InnerCloud) else np.asarray(cloud, np.float32)
+    p = np.asarray(p, np.float32)
+    if p.ndim != 2 or p.shape[1] not in (3, 5):
+        raise ValueError("cloud must be (N,3) or (N,5) float32")
+    if p.shape[1] == 3:
+        p = np.concatenate([p, np.zeros((p.shape[0], 2), np.float32)], axis=1)
+    return np.ascontiguousarray(p)
+
+
+def _filter_check(rc, what):
+    if rc == -20:
+        raise RuntimeError("staticmapping_b200: no CUDA device (no CPU fallback)")
+    if rc in (-1, -10, -11):
+        raise CheckFailure(f"{what} failed with {rc}")
+    if rc < 0:
+        raise RuntimeError(f"{what} failed with {rc}")
+    return rc
+
+
+def _init_stage(chain, stage, name, node):
+    """Interface::InitFromXmlNode (filter_interface.cc:29-60) on one stage -> ConfigsValid()."""
+    if node.tag != "filter":
+        raise CheckFailure(f"expected a <filter> node, got <{node.tag}>")
+    if node.get("name", "") != name:
+        return False
+    for p in node.findall("param"):
+        t = p.get("type")
+        rc = chain.set_param(stage, p.get("name", ""), int(t) if t is not None else 2, p.text or "")
+        if rc < 0:
+            raise CheckFailure(f"{name}: param {p.get('name')!r} (type {t}) rejected with {rc}")
+    return bool(chain.valid(stage))
+
+
+class FilterFactory:
+    """pre_processers::filter::Factory (filter_factory.cc:63-123) on the GPU: the <filters> chain of the XML config.
+    `chain` replaces the GPU backend (tests pass the serial oracle).  Unknown filter names raise CheckFailure (the
+    reference skips them), unknown parameters too (the reference CHECK-fails)."""
+
+    def __init__(self, device=0, seed=0, chain=None):
+        self._chain = chain if chain is not None else FilterChain(device)
+        self._chain.set_seed(seed)
+        self.names = []
+        self._cloud = None
+
+    def InitFromXmlText(self, text):
+        self.InitFromXmlNode(ET.fromstring(text))
+
+    def InitFromXmlNode(self, filters_node):
+        for node in filters_node.findall("filter"):
+            name = node.get("name", "")
+            stage = self._chain.add(name)
+            if stage < 0:
+                raise CheckFailure(f"filter {name!r} is not supported ({stage})")
+            _init_stage(self._chain, stage, name, node)
+            self.names.append(name)
+
+    def SetInputCloud(self, cloud):
+        self._cloud = _records(cloud)
+
+    def Filter(self):
+        """-> (M,5) float32 records of the filtered cloud.  KeptIndex() gives their chain-input indices."""
+        if self._cloud is None:
+            raise CheckFailure("FilterFactory: SetInputCloud first")
+        rc, out, kept = self._chain.filter(self._cloud)
+        _filter_check(rc, "FilterFactory::Filter")
+        self._kept = kept
+        return out
+
+    def FilterDevice(self, cloud):
+        """contiguous (N,5) float32 CUDA tensor -> ((M,5) tensor, (M,) int32 chain-input indices); the cloud never
+        leaves the device."""
+        rc, out, kept = self._chain.filter_device(cloud)
+        _filter_check(rc, "FilterFactory::FilterDevice")
+        return out, kept
+
+    def KeptIndex(self):
+        return self._kept
+
+    def StageCounts(self):
+        return self._chain.stage_counts()
+
+    def StageMs(self):
+        return self._chain.stage_ms()
+
+
+class _Filter:
+    """One pre_processers::filter::Interface (filter_interface.h) on the GPU: a one-stage chain."""
+    NAME = ""
+
+    def __init__(self, device=0, seed=0, chain=None):
+        self._chain = chain if chain is not None else FilterChain(device)
+        self._chain.set_seed(seed)
+        self._stage = _filter_check(self._chain.add(self.NAME), f"{self.NAME}()")
+        self._cloud = None
+        self._inliers = np.zeros(0, np.int64)
+        self._outliers = np.zeros(0, np.int64)
+
+    def InitFromXmlNode(self, node):
+        return _init_stage(self._chain, self._stage, self.NAME, node)
+
+    def InitFromXmlText(self, text):
+        return self.InitFromXmlNode(ET.fromstring(text))
+
+    def ConfigsValid(self):
+        return bool(self._chain.valid(self._stage))
+
+    def SetInputCloud(self, cloud):
+        self._cloud = _records(cloud)
+        self._inliers = np.zeros(0, np.int64)
+        self._outliers = np.zeros(0, np.int64)
+
+    def Filter(self):
+        """-> (M,5) float32 records; Inliers() / Outliers() are updated like the reference's."""
+        if self._cloud is None:
+            raise CheckFailure(f"{self.NAME}: SetInputCloud first")
+        rc, out, kept = self._chain.filter(self._cloud)
+        _filter_check(rc, f"{self.NAME}::Filter")
+        self._inliers = np.sort(kept[kept >= 0]).astype(np.int64)
+        self._outliers = self._outlier_set()
+        return out
+
+    def _outlier_set(self):
+        mask = np.ones(self._cloud.shape[0], bool)
+        mask[self._inliers] = False
+        return np.flatnonzero(mask).astype(np.int64)
+
+    def Inliers(self):
+        return self._inliers
+
+    def Outliers(self):
+        return self._outliers
+
+
+class Range(_Filter):
+    NAME = "Range"
+
+
+class AxisRange(_Filter):
+    NAME = "AxisRange"
+
+
+class BoundingBoxRemoval(_Filter):
+    NAME = "BoundingBoxRemoval"
+
+
+class RandomSampler(_Filter):
+    NAME = "RandomSampler"
+
+
+class RangeImage(_Filter):
+    NAME = "RangeImage"
+
+
+class GroundRemoval2(_Filter):
+    NAME = "GroundRemoval2"
+
+
+class GroundRemoval(_Filter):
+    NAME = "GroundRemoval"
+
+    def __init__(self, device=0, seed=0, chain=None):
+        super().__init__(device, seed, chain)
+        self._leaf, self._min_pts = 0.8, 10
+
+    def InitFromXmlNode(self, node):
+        ok = super().InitFromXmlNode(node)
+        for p in node.findall("param"):                 # the vanished voxels of Outliers() need these two
+            if p.get("name") == "leaf_size":
+                self._leaf = float(np.float32(float(p.text)) if p.get("type") == "1" else int(float(p.text)))
+            if p.get("name") == "min_point_num_in_voxel":
+                self._min_pts = int(float(p.text)) if p.get("type") == "1" else int(p.text)
+        return ok
+
+    def _outlier_set(self):
+        """voxels below min_point_num_in_voxel vanish: their points are neither inliers nor outliers"""
+        p = self._cloud[:, :3]
+        fin = np.isfinite(p).all(axis=1)
+        with np.errstate(invalid="ignore", over="ignore"):
+            v = np.trunc(p / np.float32(self._leaf)).astype(np.int64)
+        v[~fin] = 0
+        _, inv, cnt = np.unique(v, axis=0, return_inverse=True, return_counts=True)
+        small = (cnt[inv.reshape(-1)] < self._min_pts) & fin
+        mask = ~small
+        mask[self._inliers] = False
+        return np.flatnonzero(mask).astype(np.int64)
+
+
+class VoxelGrid(_Filter):
+    """VoxelGrid::Filter: inliers and outliers stay empty, like the reference's (FilterPrepare clears them)."""
+    NAME = "VoxelGrid"
+
+    def Filter(self):
+        out = super().Filter()
+        self._inliers = self._outliers = np.zeros(0, np.int64)
+        return out
+
+
+class StatisticRemoval(_Filter):
+    """StatisticRemoval: the identity; its body (and so its inliers / outliers) is commented out in the reference."""
+    NAME = "StatisticRemoval"
+
+    def Filter(self):
+        out = super().Filter()
+        self._inliers = self._outliers = np.zeros(0, np.int64)
+        return out
